@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- stereo pairs rendered + TSDF-fused per second (BASELINE.json's metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config C1] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config C1] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 One STEP = one stereo pair of the synthetic scene: render the left and the right view
@@ -18,6 +18,9 @@ K pairs per rank) and the timed region ends with the single NCCL sum-reduce of t
            renderer_utils.py:378-390 calls it (float frame D2H, x255 -> uint8 on the host) and the
            Open3D-0.17-equivalent CPU TSDF (oracle port, all host threads).  PNG encoding and the
            stereo network are left out (both would only slow the reference arm down).
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what the last timed step handed its caller as DIR/<name>.npy
+           (float32 / float64, see dump_outputs), so that two builds can be compared output for output on the same
+           seeded inputs.
 Prints ONE JSON line on rank 0.
 """
 from __future__ import annotations
@@ -62,14 +65,13 @@ class BenchArgs:
 
 
 def measured_peak_gbs():
-    for p in (os.path.join(ROOT, "MEASURED_PEAKS.json"), "/root/repo/MEASURED_PEAKS.json"):
-        try:
-            with open(p) as f:
-                v = json.load(f).get("hbm_gbs")
-            if v:
-                return float(v), "measured"
-        except Exception:
-            pass
+    try:
+        with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as f:
+            v = json.load(f).get("hbm_gbs")
+        if v:
+            return float(v), "measured"
+    except Exception:
+        pass
     return 6650.0, "fallback"
 
 
@@ -182,6 +184,35 @@ def workload_name(name, cfg, total_views):
 
 # ------------------------------------------------------------------------------------------------ ours
 DEFAULT_E2E_ORDER = "lagged"
+DUMP_MAX_VALUES = 1 << 20  # per dumped array (4 MB as float32): the ten arrays stay well under 64 MB together
+
+
+def _dump_values(t):
+    """Device tensor -> float32 host array; above DUMP_MAX_VALUES values, the same seeded sample of positions on every run."""
+    flat = t.reshape(-1)
+    if flat.numel() <= DUMP_MAX_VALUES:
+        return t.float().cpu().numpy()
+    pick = np.sort(np.random.default_rng(0).choice(flat.numel(), DUMP_MAX_VALUES, replace=False))
+    return flat[torch.from_numpy(pick).to(flat.device)].float().cpu().numpy()
+
+
+def dump_outputs(out_dir, out, vol):
+    """What the last timed step handed its caller: the pair's float and uint8 frames, the left view's depth and
+    transmittance, and the TSDF volume after its fusion.  Bricks are listed in lattice-index order (pool slots depend on
+    the order in which blocks opened them): volume_brick_index [n,3] (float64) and the bricks' tsdf / weight / colour."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: _dump_values(out[k]) for k in ("left", "right", "left_u8", "right_u8", "depth", "final_T")}
+    index = vol.brick_indices().cpu().numpy()
+    order = np.lexsort(index.T[::-1])
+    slots = torch.from_numpy(order).to(vol.device)
+    arrays["volume_brick_index"] = index[order].astype(np.float64)
+    bricks = vol.pool()[slots]
+    arrays["volume_tsdf"] = _dump_values(bricks[..., 0])
+    arrays["volume_weight"] = _dump_values(bricks[..., 1])
+    if vol.color is not None:
+        arrays["volume_color"] = _dump_values(vol.color.view(vol.pool_bricks, -1, 4)[slots][..., :3])
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def run_ours(args, cfg, rank, local, world):
@@ -215,6 +246,7 @@ def run_ours(args, cfg, rank, local, world):
     def step(i):
         out = renderer.render_image_pair(i, to_host=False)
         stage.integrate(out["depth"], out["left_u8"], rigs[i]["left"], final_T=out["final_T"])
+        return out
 
     # ---- calibration (untimed): per-view workload statistics for the roofline formulas
     stats = dict(Pv=[], R=[], R_ref=[], bricks=[], V_upd=[])
@@ -257,8 +289,9 @@ def run_ours(args, cfg, rank, local, world):
     barrier(world)
     ev0.record()
     host_t0 = time.perf_counter()
+    last = None
     for i in mine:
-        step(i)
+        last = step(i)
     host_enqueue_ms = 1e3 * (time.perf_counter() - host_t0) / max(K, 1)  # host time to ENQUEUE a step (no waiting)
     evr = torch.cuda.Event(enable_timing=True)
     evr.record()
@@ -274,6 +307,8 @@ def run_ours(args, cfg, rank, local, world):
     launches = int(_lib.lib().gsb_kernel_launch_count() - launches0)
     elapsed_ms = max_over_ranks(ev0.elapsed_time(ev1), world)
     value = total_views / (elapsed_ms / 1e3)
+    if args.dump_outputs and rank == 0 and last is not None:
+        dump_outputs(args.dump_outputs, last, vol)
 
     # ---- per-kernel durations: the same steps again with the two eyes serialised on one stream, every
     #      stage bracketed by CUDA events on the launching stream (in the timed loop above the eyes overlap
@@ -617,8 +652,12 @@ def main():
     ap.add_argument("--cpu-budget", type=float, default=20.0)
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak (driver contract): --steps pairs PER RANK; strong: --steps pairs in total, split over the ranks")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write the last step's outputs as DIR/<name>.npy (--impl ours)")
     ap.add_argument("--emit-depth-frames", default=None, help=argparse.SUPPRESS)  # child process of the reference arm
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs is only implemented for --impl ours")
     if args.warmup < 3:
         args.warmup = 3
     from gs2mesh_b200 import scene
@@ -641,7 +680,6 @@ def main():
         emit_depth_frames(args, cfg, local)
         return
     if args.impl == "reference":
-        args.steps = min(args.steps, 200)  # bounded: ~0.25 s of CPU TSDF per step at C1
         line = run_reference(args, cfg, rank, local, world)
     else:
         line = run_ours(args, cfg, rank, local, world)

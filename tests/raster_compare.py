@@ -5,6 +5,10 @@ A pixel is "bad" if |a-b| > 1e-4 * max(1, |b|).  The pipeline has hard threshold
 difference in expf or an FMA contraction can flip for isolated pixels (SURVEY.md section 7,
 "Branch-boundary parity"), so comparisons carry an explicit outlier budget instead of a max.
 """
+import hashlib
+import math
+import os
+
 import numpy as np
 
 TOL = 1e-4
@@ -33,6 +37,53 @@ def compare_images(a, b):
     return dict(frac_bad=float(bad.sum() / n), max_err=float(err.max()) if err.size else 0.0, n_bad=int(bad.sum()),
                 median=float(np.median(err)) if err.size else 0.0, frac_bad_rel=float(bad_rel.sum() / n),
                 max_err_rel=float(rel.max()) if rel.size else 0.0, p9999_rel=float(np.quantile(rel, 0.9999)) if rel.size else 0.0)
+
+
+def fixed_sample(n_total, n):
+    """Indices of an evenly spread, fixed sample of n of n_total values (a golden-ratio lattice, no RNG involved).
+    The first m indices of a sample of n are the sample of m, so a stored sample can be shortened without re-running."""
+    step = int(n_total * 0.6180339887498949) | 1
+    while math.gcd(step, n_total) != 1:
+        step += 2
+    return (np.arange(min(n, n_total), dtype=np.int64) * step) % n_total
+
+
+def digest(*arrays):
+    """sha256 over dtype, shape and bytes: stands in for an exact comparison with an array too large to store."""
+    h = hashlib.sha256()
+    for a in arrays:
+        a = np.ascontiguousarray(a)
+        h.update(f"{a.dtype.str}{a.shape}".encode())
+        h.update(a.tobytes())
+    return h.hexdigest()
+
+
+def inputs_digest(*arrays):
+    """digest() of rasterizer inputs as the float32 values the kernels receive."""
+    return digest(*(np.ascontiguousarray(a, dtype=np.float32).reshape(-1) for a in arrays))
+
+
+REF_GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def load_ref_golden(file_name, key, inputs_sha256):
+    """One case of the reference rasterizer's stored outputs (tests/golden/make_ref_parity_golden.py): exact outputs as
+    digests (`*_sha256`), images as the fixed_sample() of their pixels.  Fails if the case's inputs are no longer the ones
+    the outputs were recorded for."""
+    with np.load(os.path.join(REF_GOLDEN_DIR, file_name)) as z:
+        case = {k[len(key) + 2:]: z[k] for k in z.files if k.startswith(key + "__")}
+    assert case, f"no case {key} in tests/golden/{file_name}"
+    for k in [k for k in case if k.endswith("_sha256")]:
+        case[k] = str(case[k])
+    assert case["inputs_sha256"] == inputs_sha256, f"inputs of {key} differ from those tests/golden/{file_name} was made from"
+    return case
+
+
+def sample_image(img, n):
+    """[C,H,W] or [H,W] -> the fixed_sample() of n pixels, [C,n] or [n]."""
+    img = np.asarray(img)
+    flat = img.reshape(img.shape[0], -1) if img.ndim == 3 else img.reshape(-1)
+    return flat[..., fixed_sample(flat.shape[-1], n)]
 
 
 def load_golden_case(path):

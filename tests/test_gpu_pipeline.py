@@ -234,6 +234,13 @@ FULL_SIZE_CASES = {
 # error 2.9e-3; full-precision expf kernel: no value outside, worst error 2.4e-7), plus a ceiling on any single outlier.
 FULL_SIZE_BUDGET = {"ex2": 4e-5, "expf": 1e-6}
 FULL_SIZE_MAX_ERR = {"ex2": 3e-2, "expf": 3e-6}
+FULL_SIZE_VIEW = 3  # the stereo pair of the 8-view rig the full-size cases render
+
+
+def full_size_inputs_sha256(cloud, camera_record):
+    from tests.raster_compare import inputs_digest
+
+    return inputs_digest(cloud.xyz, cloud.opacity, cloud.features, cloud.scaling, cloud.rotation, camera_record)
 
 
 def _record_observed(name, payload):
@@ -257,13 +264,15 @@ def _record_observed(name, payload):
 @pytest.mark.parametrize("case", list(FULL_SIZE_CASES))
 def test_full_size_parity_vs_reference_binary_and_oracle(oracle, gsb_lib, cuda_device, case):
     """BASELINE configs C1..C4 at full size: the rendered frame against the UNMODIFIED reference rasterizer (sm_100a
-    build) on the same tensors, and the fused TSDF bricks against the Open3D restatement on the same depth."""
+    build) on the same tensors, and the fused TSDF bricks against the Open3D restatement on the same depth.  The
+    reference's frames were recorded on a B200 (tests/golden/make_ref_parity_golden.py): compared on a fixed sample of
+    their pixels, the full-precision transmittance frame bit for bit through its digest."""
     import torch
 
     from gs2mesh_b200 import _lib
     from gs2mesh_b200.renderer import Renderer
     from gs2mesh_b200.tsdf import TSDF
-    from tests.raster_compare import compare_images
+    from tests.raster_compare import compare_images, digest, load_ref_golden, sample_image
 
     cfg = FULL_SIZE_CASES[case]
     W, H = cfg["width"], cfg["height"]
@@ -281,25 +290,25 @@ def test_full_size_parity_vs_reference_binary_and_oracle(oracle, gsb_lib, cuda_d
     r = Renderer.from_scene(rigs, baseline, cloud, args=A(), device=str(cuda_device))
     r.prepare_renderer()
     observed = {}
-    if oracle.ref_available():
-        for side in (0, 1):
-            rec = r._camera_table[3, side]
-            vt = r._views[3][side]
-            ref = oracle.ref_forward_torch(r.means3D, r.opacity, rec[0:16], rec[16:32], rec[32:35], W, H, vt.tan_fovx, vt.tan_fovy,
-                                           r.background, shs=r.shs, scales=r.scales, rotations=r.rotations, sh_degree=3)
-            for tag, flags in (("expf", _lib.RASTER_EXACT_TILE_CULL), ("ex2", _lib.RASTER_EXACT_TILE_CULL | _lib.RASTER_FAST_EXP)):
-                ours = r.render_view(3, side, want_depth=True, want_counts=True, flags=flags)
-                cmp = compare_images(ours["color"].cpu().numpy(), ref["color"].cpu().numpy())
-                cmpT = compare_images(ours["final_T"].cpu().numpy(), ref["final_T"].cpu().numpy())
-                observed[f"side{side}_{tag}"] = dict(color=cmp, final_T=cmpT, num_rendered_ref=int(ref["num_rendered"]),
-                                                     instances_binned=int(ours["counts"][0]))
-                _record_observed(case, observed)
-                assert cmp["frac_bad_rel"] <= FULL_SIZE_BUDGET[tag] and cmp["median"] <= 1e-6, (side, tag, cmp)
-                assert cmp["max_err"] <= FULL_SIZE_MAX_ERR[tag], (side, tag, cmp)
-                assert cmpT["frac_bad_rel"] <= FULL_SIZE_BUDGET[tag] and cmpT["max_err"] <= FULL_SIZE_MAX_ERR[tag], (side, tag, cmpT)
-                if tag == "expf":  # the reference's own exponent expression + expf: transmittance bit for bit
-                    assert cmpT["max_err"] == 0.0, (side, cmpT)
-                assert int(ours["counts"][1]) == ref["num_rendered"]  # the reference's instance count, exactly
+    for side in (0, 1):
+        rec = r._camera_table[FULL_SIZE_VIEW, side].cpu().numpy()
+        ref = load_ref_golden("ref_raster_full_size.npz", f"{case}-side{side}", full_size_inputs_sha256(cloud, rec))
+        n = ref["final_T"].size
+        for tag, flags in (("expf", _lib.RASTER_EXACT_TILE_CULL), ("ex2", _lib.RASTER_EXACT_TILE_CULL | _lib.RASTER_FAST_EXP)):
+            ours = r.render_view(FULL_SIZE_VIEW, side, want_depth=True, want_counts=True, flags=flags)
+            ours_T = ours["final_T"].cpu().numpy()
+            cmp = compare_images(sample_image(ours["color"].cpu().numpy(), n), ref["color"])
+            cmpT = compare_images(sample_image(ours_T, n), ref["final_T"])
+            observed[f"side{side}_{tag}"] = dict(color=cmp, final_T=cmpT, num_rendered_ref=int(ref["num_rendered"]),
+                                                 instances_binned=int(ours["counts"][0]))
+            _record_observed(case, observed)
+            assert cmp["frac_bad_rel"] <= FULL_SIZE_BUDGET[tag] and cmp["median"] <= 1e-6, (side, tag, cmp)
+            assert cmp["max_err"] <= FULL_SIZE_MAX_ERR[tag], (side, tag, cmp)
+            assert cmpT["frac_bad_rel"] <= FULL_SIZE_BUDGET[tag] and cmpT["max_err"] <= FULL_SIZE_MAX_ERR[tag], (side, tag, cmpT)
+            if tag == "expf":  # the reference's own exponent expression + expf: transmittance bit for bit, whole frame
+                assert cmpT["max_err"] == 0.0, (side, cmpT)
+                assert digest(ours_T + np.float32(0)) == ref["final_T_sha256"], side
+            assert int(ours["counts"][1]) == ref["num_rendered"]  # the reference's instance count, exactly
 
     pair = r.render_image_pair(3, to_host=False)
     stage = TSDF(r, None, A(), case, window_resolution=res)

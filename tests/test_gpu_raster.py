@@ -1,5 +1,7 @@
 """GPU parity tests of the rasterizer: CUDA path (through the C ABI) vs the CPU oracle and vs the
-UNMODIFIED reference rasterizer built for sm_100a (oracle/_ref/libref_dgr.so), same seeded inputs.
+UNMODIFIED reference rasterizer built for sm_100a, same seeded inputs.  The reference's outputs were recorded on a B200
+(tests/golden/make_ref_parity_golden.py -> tests/golden/ref_raster_views.npz): exact outputs as digests, images as a
+fixed sample of their pixels.
 
 Tolerance (north_star): 1e-4 relative fp32 per pixel, with an outlier budget for pixels where a
 hard threshold of the algorithm flips (see tests/raster_compare.py).  Integer outputs (radii,
@@ -12,9 +14,12 @@ import pytest
 
 from gs2mesh_b200 import camera as cam
 from gs2mesh_b200 import scene
-from tests.raster_compare import compare_images
+from tests.raster_compare import compare_images, digest, fixed_sample, inputs_digest, load_ref_golden, sample_image
 
 pytestmark = pytest.mark.gpu
+
+REF_CASES = [(3000, 320, 240, 0), (10000, 640, 480, 1), (777, 250, 130, 2)]  # (num_points, W, H, seed)
+PINNED_CASE = (4000, 320, 240, 5)
 
 BUDGET = 1e-4  # fraction of values allowed outside 1e-4 (hard thresholds flip on rounding); on these small frames one flipped
                # pixel is already 4e-6 .. 1e-5 of the values.  Full-size frames: tests/test_gpu_pipeline.py (4e-5, observed 4e-6)
@@ -52,16 +57,19 @@ def _ours(dev, inp, flags=None, **kw):
     return {k: (v.cpu().numpy() if v is not None else None) for k, v in out.items()}
 
 
-def _ref(oracle, dev, inp):
-    import torch
+def case_key(num_points, W, H, seed):
+    return f"{num_points}-{W}-{H}-{seed}"
 
-    t = lambda a: None if a is None else torch.as_tensor(np.ascontiguousarray(a, dtype=np.float32)).to(dev)
-    out = oracle.ref_forward_torch(t(inp["means3D"]), t(inp["opacities"]).reshape(-1), t(inp["view"]), t(inp["proj"]), t(inp["campos"]),
-                                   inp["W"], inp["H"], inp["tan_fovx"], inp["tan_fovy"], t(inp["bg"]), shs=t(inp.get("shs")),
-                                   colors_precomp=t(inp.get("colors_precomp")), scales=t(inp.get("scales")),
-                                   rotations=t(inp.get("rotations")), cov3D_precomp=t(inp.get("cov3D_precomp")),
-                                   sh_degree=inp["sh_degree"], scale_modifier=inp["scale_modifier"], want_geometry=True)
-    return {k: (v.cpu().numpy() if hasattr(v, "cpu") else v) for k, v in out.items()}
+
+def inputs_sha256(inp):
+    return inputs_digest(inp["means3D"], inp["opacities"], inp["shs"], inp["scales"], inp["rotations"], inp["view"], inp["proj"],
+                         inp["campos"], inp["bg"], [inp["W"], inp["H"], inp["tan_fovx"], inp["tan_fovy"], inp["sh_degree"],
+                                                    inp["scale_modifier"]])
+
+
+def _ref(num_points, W, H, seed, inp):
+    """The reference rasterizer's recorded outputs for this case (see the module docstring)."""
+    return load_ref_golden("ref_raster_views.npz", case_key(num_points, W, H, seed), inputs_sha256(inp))
 
 
 def _assert_parity(a, b, what, budget=BUDGET):
@@ -92,45 +100,44 @@ def test_cuda_matches_cpu_oracle(oracle, gsb_lib, cuda_device, num_points, W, H,
     _assert_parity(ours["depth"], o["depth"], "depth")
 
 
-@pytest.mark.parametrize("num_points,W,H,seed", [(3000, 320, 240, 0), (10000, 640, 480, 1), (777, 250, 130, 2)])
-def test_cuda_matches_reference_rasterizer(oracle, gsb_lib, cuda_device, num_points, W, H, seed):
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref/libref_dgr.so not built")
+@pytest.mark.parametrize("num_points,W,H,seed", REF_CASES)
+def test_cuda_matches_reference_rasterizer(gsb_lib, cuda_device, num_points, W, H, seed):
     g, vt = _case(num_points, W, H, seed)
     inp = _np_inputs(g, vt)
-    ref = _ref(oracle, cuda_device, inp)
+    ref = _ref(num_points, W, H, seed, inp)
+    n = ref["final_T"].size
     from gs2mesh_b200 import _lib
 
     rect = _ours(cuda_device, inp, flags=0)  # reference rectangle binning
-    np.testing.assert_array_equal(rect["radii"], ref["radii"])
+    assert digest(rect["radii"]) == ref["radii_sha256"]
     assert int(rect["counts"][0]) == ref["num_rendered"] == int(rect["counts"][1])
-    _assert_parity(rect["color"], ref["color"], "color(rect)")
-    _assert_parity(rect["final_T"], ref["final_T"], "final_T(rect)")
+    _assert_parity(sample_image(rect["color"], n), ref["color"], "color(rect)")
+    _assert_parity(sample_image(rect["final_T"], n), ref["final_T"], "final_T(rect)")
     ours = _ours(cuda_device, inp, flags=_lib.RASTER_EXACT_TILE_CULL)
-    _assert_parity(ours["color"], ref["color"], "color(exact)")
+    _assert_parity(sample_image(ours["color"], n), ref["color"], "color(exact)")
     assert int(ours["counts"][1]) == ref["num_rendered"]
 
 
-def test_oracle_is_pinned_by_reference_rasterizer(oracle, cuda_device):
+def test_oracle_is_pinned_by_reference_rasterizer(oracle):
     """Pins the CPU restatement itself: oracle vs the reference binary on the same inputs,
-    per-Gaussian intermediates included."""
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref/libref_dgr.so not built")
-    g, vt = _case(4000, 320, 240, seed=5)
+    per-Gaussian intermediates included (for a fixed sample of the visible Gaussians)."""
+    g, vt = _case(*PINNED_CASE[:3], seed=PINNED_CASE[3])
     inp = _np_inputs(g, vt)
-    ref = _ref(oracle, cuda_device, inp)
+    ref = _ref(*PINNED_CASE, inp)
     pre = oracle.preprocess(g.xyz, g.opacity, vt.world_view, vt.full_proj, vt.cam_center, vt.width, vt.height, vt.tan_fovx,
                             vt.tan_fovy, shs=g.features, scales=g.scaling, rotations=g.rotation)
-    vis = ref["radii"] > 0
-    np.testing.assert_array_equal(pre["radii"], ref["radii"])
-    np.testing.assert_array_equal(pre["tiles_touched"], ref["tiles_touched"].astype(np.uint32))
-    np.testing.assert_allclose(pre["depths"][vis], ref["depths"][vis], rtol=1e-6)
-    np.testing.assert_allclose(pre["xy"][vis], ref["xy"][vis], rtol=1e-5, atol=1e-4)
-    np.testing.assert_allclose(pre["conic_opacity"][vis], ref["conic_opacity"][vis], rtol=2e-4, atol=1e-6)
-    np.testing.assert_allclose(pre["rgb"][vis], ref["rgb"][vis], rtol=1e-5, atol=2e-6)
+    assert digest(pre["radii"]) == ref["radii_sha256"]
+    assert digest(pre["tiles_touched"]) == ref["tiles_touched_sha256"]
+    vis = np.flatnonzero(pre["radii"] > 0)  # == the reference's visible set: the radii are equal
+    gi = vis[fixed_sample(len(vis), len(ref["depths"]))]
+    np.testing.assert_allclose(pre["depths"][gi], ref["depths"], rtol=1e-6)
+    np.testing.assert_allclose(pre["xy"][gi], ref["xy"], rtol=1e-5, atol=1e-4)
+    np.testing.assert_allclose(pre["conic_opacity"][gi], ref["conic_opacity"], rtol=2e-4, atol=1e-6)
+    np.testing.assert_allclose(pre["rgb"][gi], ref["rgb"], rtol=1e-5, atol=2e-6)
     o, of = _oracle_best(oracle, inp)
     assert o["num_rendered"] == ref["num_rendered"]
-    best = min((compare_images(x["color"], ref["color"]) for x in (o, of)), key=lambda r: r["frac_bad"])
+    n = ref["final_T"].size
+    best = min((compare_images(sample_image(x["color"], n), ref["color"]) for x in (o, of)), key=lambda r: r["frac_bad"])
     assert best["frac_bad"] <= BUDGET, best
 
 
@@ -237,10 +244,10 @@ def test_fast_exp_stays_inside_parity_budget(oracle, gsb_lib, cuda_device):
         exact = _ours(cuda_device, inp, flags=_lib.RASTER_EXACT_TILE_CULL)
         r = compare_images(fast["color"], exact["color"])
         assert r["frac_bad"] <= BUDGET and r["median"] <= 1e-6, r
-        if oracle.ref_available():
-            ref = _ref(oracle, cuda_device, inp)
-            _assert_parity(fast["color"], ref["color"], "fast-exp color vs reference")
-            _assert_parity(fast["final_T"], ref["final_T"], "fast-exp final_T vs reference")
+        ref = _ref(n, W, H, seed, inp)
+        k = ref["final_T"].size
+        _assert_parity(sample_image(fast["color"], k), ref["color"], "fast-exp color vs reference")
+        _assert_parity(sample_image(fast["final_T"], k), ref["final_T"], "fast-exp final_T vs reference")
         o = oracle.forward(**inp)
         _assert_parity(fast["depth"], o["depth"], "fast-exp depth vs oracle")
 
